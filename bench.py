@@ -40,6 +40,8 @@ STRIDE = 76544
 MUL = 65521
 TEXT_FILES = ("alice29.txt", "asyoulik.txt", "lcet10.txt", "plrabn12.txt")
 METRIC = "uncompressed GB/s, raw 64KB-block compress+decompress round trip"
+DUMP_SAMPLE, DUMP_SEED = 32, 0       # --dump-outputs: blocks of the last wave whose bytes are written, and their seed
+DUMP_LIMIT = 64 << 20
 
 
 def load_text():
@@ -352,6 +354,9 @@ def run_ours(args, rank, local_rank, world):
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = L.sb_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        lo = (nwaves - 1) * wave
+        dump_outputs(args.dump_outputs, t_clen, t_c, t_out, t_dlen, t_st, lo, blocks - lo)
 
     # max over ranks of the device-timed step
     tot = torch.tensor([ms_c + ms_d, ms_c, ms_d], dtype=torch.float64, device=dev)
@@ -427,6 +432,36 @@ def run_ours(args, rank, local_rank, world):
         from oracle import oracle as orc
         line["cpu_baseline"], _ = cpu_baseline_report(orc, text, 12.0)
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, t_clen, t_c, t_out, t_dlen, t_st, lo, cnt):
+    """--dump-outputs: what the last timed step handed back, as <name>.npy in float32 (bytes, lengths) or float64
+    (status records), so that two builds can be compared array for array. The compressed length covers every block;
+    the staging buffers hold only the last wave (blocks lo .. lo+cnt-1), whose lengths and statuses are written in
+    full and whose bytes are written for a fixed seeded sample of DUMP_SAMPLE blocks (compressed slots padded with -1
+    past the stream's end, where the slot holds no output)."""
+    import numpy as np
+    clen = t_clen.cpu().numpy()
+    pick = np.sort(np.random.default_rng(DUMP_SEED).choice(cnt, size=min(DUMP_SAMPLE, cnt), replace=False))
+    comp = np.full((len(pick), STRIDE), -1.0, dtype=np.float32)
+    back = np.empty((len(pick), BLOCK), dtype=np.float32)
+    for k, i in enumerate(pick):
+        n = int(clen[lo + i])
+        comp[k, :n] = t_c[i * STRIDE:i * STRIDE + n].cpu().numpy()
+        back[k] = t_out[i * BLOCK:(i + 1) * BLOCK].cpu().numpy()
+    arrays = {
+        "compressed_len": clen.astype(np.float32),
+        "sample_block": (lo + pick).astype(np.float64),
+        "compressed_sample": comp,
+        "decompressed_len": t_dlen[:cnt].cpu().numpy().astype(np.float32),
+        "decompressed_sample": back,
+        "decompress_status": t_st.view(-1, 4)[:cnt].cpu().numpy().astype(np.float64),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, "--dump-outputs would write %d bytes" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_e2e(args, snap, L, torch, dev, t_in, t_clen, rank, world):
@@ -882,7 +917,11 @@ def main():
     ap.add_argument("--urls-gib", type=float, default=64.0)
     ap.add_argument("--gib", type=float, default=None)
     ap.add_argument("--wave-gib", type=float, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="text-roundtrip: after the timed steps, write what the last step computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "text-roundtrip"):
+        ap.error("--dump-outputs applies to --impl ours --workload text-roundtrip")
     if args.warmup < 3 and args.workload != "frame-shard":
         args.warmup = 3          # frame-shard steps are whole-stream passes (hundreds of waves each): --warmup 1 is accepted there
     rank = int(os.environ.get("RANK", "0"))
