@@ -183,6 +183,45 @@ int sb_frame_decode_device(const uint8_t* d_in, uint64_t n, uint8_t* d_out, uint
                            const uint64_t* d_chunk_offs, uint32_t nchunks, uint32_t flags,
                            sb_frame_result* result, void* stream, sb_error* err);
 
+/* ---- batches of raw streams of any size (units above 64KB) ----------------
+ * Unit i = d_in_ptrs[i][0 .. d_in_lens[i]) (device pointer and length arrays); each becomes exactly
+ * Encoder::compress(unit) (src/compress.rs:99-154): one varint of the unit's length, then its 64KB blocks.
+ * The library lays the streams out back to back in d_out[0 .. cap) and reports where: d_out_offs receives count+1
+ * entries (d_out_offs[count] = total bytes). The whole batch is one launch sequence on `stream` -- no allocation, no
+ * host synchronisation; the outcome lands in *d_result (device): status, bytes = total, nchunks = 64KB blocks.
+ *   total_in: a host-side upper bound on the sum of the lengths; it sizes the scratch and the launch
+ *     (units + total_in/65536 block slots). A sum above it is SB_E_INVALID{a=sum, b=total_in} and nothing is written.
+ *   A unit with sb_max_compress_len(len) == 0 is refused with TooBig{given=len, max=2^32-1} and gets an empty
+ *     stream (d_out_offs[i+1] == d_out_offs[i]); the other units are compressed. d_result reports the first such unit.
+ *   Output larger than cap: nothing is written, d_result (and every status) is BufferTooSmall{given=cap, min=total};
+ *     the offsets are still reported, so a caller can size a retry. sum(sb_max_compress_len(len)) is always enough.
+ *   d_statuses (may be NULL): per unit Ok / TooBig, or the call's failure.
+ *   scratch: device memory of at least sb_compress_streams_scratch_bytes(count, total_in). */
+uint64_t sb_compress_streams_scratch_bytes(uint32_t count, uint64_t total_in);
+int sb_compress_streams_device_ws(const uint8_t* const* d_in_ptrs, const uint64_t* d_in_lens, uint32_t count,
+                                  uint64_t total_in, uint8_t* d_out, uint64_t cap, uint64_t* d_out_offs,
+                                  sb_error* d_statuses, sb_frame_result* d_result,
+                                  void* scratch, uint64_t scratch_bytes, void* stream, sb_error* err);
+/* Host buffers: unit i = in_base[in_offs[i] .. +in_lens[i]), streams packed back to back into out_base[0 .. out_cap)
+ * with out_offs[0..count] reported (count+1 entries). Pipelined waves like sb_compress_batch_host_packed; a unit larger
+ * than a wave gets a wave of its own. Any unit with sb_max_compress_len(len) == 0 fails the call up front with TooBig
+ * for the first such unit. For sb_reserve, a wave of this call counts its units plus the 64KB blocks they span. */
+int sb_compress_streams_host_packed(const uint8_t* in_base, const uint64_t* in_offs, const uint64_t* in_lens, size_t count,
+                                    uint8_t* out_base, uint64_t out_cap, uint64_t* out_offs, sb_error* err);
+/* Unit i = one raw stream d_in_ptrs[i][0 .. d_in_lens[i]) (device). Output sizes come from the streams' own varint
+ * headers (0 for an unusable header) and are laid out back to back in d_out (d_out_offs: count+1 entries);
+ * d_statuses[i] (required) = Decoder::decompress's result for unit i (src/decompress.rs:75-95), decoded by K2 exactly
+ * as sb_decompress_batch_device does; a stream longer than 2^32-1 bytes is SB_E_INVALID for that unit, as in
+ * sb_decompress. If the total exceeds cap no unit is decoded, and d_result and every status are
+ * BufferTooSmall{given=cap, min=total}. Otherwise d_result = the first failing unit's status (or Ok), bytes = total,
+ * nchunks = count. Stream ordered, no allocation, no host synchronisation.
+ *   scratch: device memory of at least sb_decompress_streams_scratch_bytes(count). */
+uint64_t sb_decompress_streams_scratch_bytes(uint32_t count);
+int sb_decompress_streams_device_ws(const uint8_t* const* d_in_ptrs, const uint64_t* d_in_lens, uint32_t count,
+                                    uint8_t* d_out, uint64_t cap, uint64_t* d_out_offs, sb_error* d_statuses,
+                                    sb_frame_result* d_result, void* scratch, uint64_t scratch_bytes,
+                                    void* stream, sb_error* err);
+
 /* ---- resources -------------------------------------------------------------
  * The host entry points keep grow-only per-device pools (device staging, pinned
  * descriptors, streams, events): the first calls size them, the steady state

@@ -38,6 +38,8 @@ SYMBOLS = [
     "sb_frame_max_len", "sb_frame_encode", "sb_frame_encode_ex", "sb_frame_decode", "sb_frame_encode_device",
     "sb_frame_encode_scratch_bytes", "sb_frame_encode_device_ws", "sb_frame_decode_scratch_bytes",
     "sb_frame_decode_device_ws", "sb_frame_decode_device", "sb_reserve", "sb_alloc_count",
+    "sb_compress_streams_scratch_bytes", "sb_compress_streams_device_ws", "sb_compress_streams_host_packed",
+    "sb_decompress_streams_scratch_bytes", "sb_decompress_streams_device_ws",
     "sb_bind_host_thread_to_device_numa",
     "sb_launch_count", "sb_generate_blocks_device", "sb_version",
     "snappy_compress", "snappy_uncompress", "snappy_max_compressed_length", "snappy_uncompressed_length",
@@ -86,6 +88,14 @@ def lib():
                                             C.c_uint32, vp, ep]
     L.sb_frame_decode_device.argtypes = [vp, C.c_uint64, vp, C.c_uint64, vp, C.c_uint32, C.c_uint32,
                                          C.POINTER(SbFrameResult), vp, ep]
+    L.sb_compress_streams_scratch_bytes.restype = C.c_uint64
+    L.sb_compress_streams_scratch_bytes.argtypes = [C.c_uint32, C.c_uint64]
+    L.sb_compress_streams_device_ws.argtypes = [vp, vp, C.c_uint32, C.c_uint64, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint64,
+                                                vp, ep]
+    L.sb_compress_streams_host_packed.argtypes = [vp, vp, vp, sz, vp, C.c_uint64, vp, ep]
+    L.sb_decompress_streams_scratch_bytes.restype = C.c_uint64
+    L.sb_decompress_streams_scratch_bytes.argtypes = [C.c_uint32]
+    L.sb_decompress_streams_device_ws.argtypes = [vp, vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint64, vp, ep]
     L.sb_reserve.argtypes = [sz, sz, sz, ep]
     L.sb_alloc_count.restype = C.c_uint64
     L.sb_bind_host_thread_to_device_numa.argtypes = [C.c_int]

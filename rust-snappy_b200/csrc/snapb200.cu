@@ -19,6 +19,7 @@
 #include "k3_crc32c.cuh"
 #include "k4_frame.cuh"
 #include "k5_frame_decode.cuh"
+#include "k7_streams.cuh"
 
 namespace {
 
@@ -46,6 +47,17 @@ __global__ void __launch_bounds__(1024) k5_scan_tiles_kernel(sbk::DecodePlan p) 
 __global__ void __launch_bounds__(128) k5_decode_kernel(sbk::DecodePlan p) { sbk::k5_decode_body(p); }
 __global__ void __launch_bounds__(32) k5_finish_kernel(sbk::DecodePlan p) { sbk::k5_finish_body(p); }
 __global__ void __launch_bounds__(256) k6_generate_kernel(sbk::GenPlan g) { sbk::k6_generate_body(g); }
+__global__ void __launch_bounds__(1024) k7_plan_kernel(sbk::StreamsPlan p) { sbk::k7_plan_body(p); }
+__global__ void __launch_bounds__(1024) k7_unit_tiles_kernel(sbk::StreamsPlan p) { sbk::k7_unit_tiles_body(p); }
+__global__ void __launch_bounds__(256) k7_expand_kernel(sbk::StreamsPlan p) { sbk::k7_expand_body(p); }
+__global__ void __launch_bounds__(1024) k7_item_scan_kernel(sbk::StreamsPlan p) { sbk::k7_item_scan_body(p); }
+__global__ void __launch_bounds__(1024) k7_item_tiles_kernel(sbk::StreamsPlan p) { sbk::k7_item_tiles_body(p); }
+__global__ void __launch_bounds__(256) k7_gather_kernel(sbk::StreamsPlan p) { sbk::k7_gather_body(p); }
+__global__ void __launch_bounds__(1024) k7_dplan_kernel(sbk::StreamsDecPlan p) { sbk::k7_dplan_body(p); }
+__global__ void __launch_bounds__(1024) k7_dtiles_kernel(sbk::StreamsDecPlan p) { sbk::k7_dtiles_body(p); }
+__global__ void __launch_bounds__(256) k7_dfill_kernel(sbk::StreamsDecPlan p) { sbk::k7_dfill_body(p); }
+__global__ void __launch_bounds__(256) k7_dfinish_kernel(sbk::StreamsDecPlan p) { sbk::k7_dfinish_body(p); }
+__global__ void __launch_bounds__(32) k7_dresult_kernel(sbk::StreamsDecPlan p) { sbk::k7_dresult_body(p); }
 
 std::atomic<uint64_t> g_launches{0};
 std::atomic<uint64_t> g_allocs{0};     // cudaMalloc / cudaHostAlloc / event + stream creations since load
@@ -95,6 +107,7 @@ struct Lane {
     cudaStream_t s_compute = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_k[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};   // host-batch pipeline
     DevBuf in[2], slots[2], compact[2], lens[2], status[2], ptrs_in[2], ptrs_out[2], caps[2], ws[2];
+    DevBuf sws[2];   // compress lane: everything of a raw-streams wave besides the K1 slots
     void* pinned[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // pinned staging: [0,1] descriptors in, [2,3] results out, [4] scalar results
     size_t pinned_cap[5] = {0, 0, 0, 0, 0};
     std::mutex mu;
@@ -377,6 +390,61 @@ int decode_payload_phase(Ctx& c, const sbk::DecodePlan& p, cudaStream_t st, sb_e
     return 0;
 }
 
+// ---- batches of raw streams of any size (K7 around K1 / K2)
+// grid of a grid-stride kernel over `work` items, `per` items per CTA, at most `most` CTAs
+unsigned grid_for(uint64_t work, unsigned per, unsigned most) {
+    const uint64_t g = (work + per - 1) / per;
+    return g == 0 ? 1u : g > most ? most : (unsigned)g;
+}
+// p: caller arrays, slots and meta carved; no host synchronisation
+int compress_streams_run(Ctx& c, const sbk::StreamsPlan& p, cudaStream_t st, sb_error* err) {
+    CK(cudaMemsetAsync(p.ctl, 0, sizeof(sbk::StreamsCtl), st));
+    CK(cudaMemsetAsync(&p.ctl->first_bad, 0xFF, 4, st));
+    const unsigned utiles = (p.count + sbk::K4_TILE - 1) / sbk::K4_TILE, itiles = (p.max_items + sbk::K4_TILE - 1) / sbk::K4_TILE;
+    k7_plan_kernel<<<utiles ? utiles : 1, sbk::K4_TILE, 32 * sizeof(uint32_t), st>>>(p);
+    k7_unit_tiles_kernel<<<1, 1024, 1024 * sizeof(uint64_t), st>>>(p);
+    k7_expand_kernel<<<grid_for(p.max_items, 256, 16 * c.sms), 256, 0, st>>>(p);
+    g_launches += 3;
+    CK(cudaGetLastError());
+    sb_batch b;
+    memset(&b, 0, sizeof b);
+    b.in_ptrs = p.item_ptr; b.in_lens = p.item_len;
+    b.out_base = p.slots; b.out_stride = sbk::kSlotStride; b.out_cap_uniform = sbk::kSlotStride;
+    b.out_lens = p.clens; b.count = p.max_items;
+    int rc = launch_k1(c, b, 0u, nullptr, st, err);   // block bodies only: the unit's varint is written by the gather
+    if (rc) return rc;
+    k7_item_scan_kernel<<<itiles ? itiles : 1, sbk::K4_TILE, 32 * sizeof(uint32_t), st>>>(p);
+    k7_item_tiles_kernel<<<1, 1024, 1024 * sizeof(uint64_t), st>>>(p);
+    const uint64_t most = p.max_items > p.count ? p.max_items : p.count;
+    k7_gather_kernel<<<grid_for(most, 8, 8 * c.sms), 256, 0, st>>>(p);
+    g_launches += 3;
+    CK(cudaGetLastError());
+    return 0;
+}
+int decompress_streams_run(Ctx& c, const sbk::StreamsDecPlan& p, cudaStream_t st, sb_error* err) {
+    CK(cudaMemsetAsync(&p.ctl->first_bad, 0xFF, 4, st));
+    const unsigned tiles = (p.count + sbk::K4_TILE - 1) / sbk::K4_TILE;
+    k7_dplan_kernel<<<tiles ? tiles : 1, sbk::K4_TILE, 32 * sizeof(uint64_t), st>>>(p);
+    k7_dtiles_kernel<<<1, 1024, 1024 * sizeof(uint64_t), st>>>(p);
+    k7_dfill_kernel<<<grid_for(p.count, 256, 16 * c.sms), 256, 0, st>>>(p);
+    g_launches += 3;
+    CK(cudaGetLastError());
+    sb_batch b;
+    memset(&b, 0, sizeof b);
+    b.in_ptrs = p.in_ptrs; b.in_lens = p.k2_in_lens;
+    b.out_ptrs = p.k2_out_ptrs; b.out_caps = p.k2_out_caps;
+    b.out_lens = p.k2_out_lens; b.statuses = p.statuses; b.count = p.count;
+    int rc = launch_k2(c, b, st, err);
+    if (rc) return rc;
+    k7_dfinish_kernel<<<grid_for(p.count, 256, 16 * c.sms), 256, 0, st>>>(p);
+    k7_dresult_kernel<<<1, 32, 0, st>>>(p);
+    g_launches += 2;
+    CK(cudaGetLastError());
+    return 0;
+}
+uint64_t streams_max_items(uint32_t count, uint64_t total_in) { return (uint64_t)count + total_in / SB_MAX_BLOCK; }
+uint64_t streams_slots_bytes(uint64_t max_items) { return align_up(max_items * (uint64_t)sbk::kSlotStride, 256); }
+
 }  // namespace
 
 // =========================================================================
@@ -451,6 +519,7 @@ int sb_reserve(size_t wave_units, size_t wave_in_bytes, size_t wave_out_bytes, s
             CK(l.ptrs_in[b].need(wave_units * 8 + 8));
             CK(l.ptrs_out[b].need(wave_units * 8 + 8));
             CK(l.ws[b].need(align_up((wave_units / sbk::K4_TILE + 3) * 8, 256) + align_up((wave_units + 1) * 8, 256) + 1024));
+            if (ln == LANE_ENC) CK(l.sws[b].need(sbk::k7_meta_bytes(wave_units, wave_units)));
             rc = need_pinned(l, b, wave_units * 24 + 64, err); if (rc) return rc;
             rc = need_pinned(l, 2 + b, wave_units * (4 + sizeof(sb_error)) + 64, err); if (rc) return rc;
         }
@@ -630,7 +699,9 @@ const size_t WAVE_BYTES = (size_t)1 << 30;
 
 struct Wave { size_t first, count; uint64_t in_bytes; };
 
-std::vector<Wave> plan_waves(const uint32_t* in_lens, size_t count, const uint32_t* out_caps) {
+extern "C++" {
+template <class Len>   // uint32_t: 64KB units; uint64_t: raw streams of any size
+std::vector<Wave> plan_waves(const Len* in_lens, size_t count, const uint32_t* out_caps) {
     std::vector<Wave> w;
     size_t i = 0;
     while (i < count) {
@@ -647,6 +718,7 @@ std::vector<Wave> plan_waves(const uint32_t* in_lens, size_t count, const uint32
     }
     return w;
 }
+}  // extern "C++"
 
 // Shared body of sb_compress_batch_host (caller's offsets) and sb_compress_batch_host_packed (the library packs the
 // streams back to back and REPORTS the offsets: a caller cannot know compressed sizes in advance).
@@ -886,6 +958,149 @@ int sb_decompress_batch_host(const uint8_t* in_base, const uint64_t* in_offs, co
         }
         CK(cudaEventRecord(l.ev_out[b], l.s_d2h));
     }
+    CK(cudaStreamSynchronize(l.s_d2h));
+    CK(cudaStreamSynchronize(l.s_compute));
+    ok(err);
+    return 0;
+}
+
+// ------------------------------------------------------- batches of raw streams
+uint64_t sb_compress_streams_scratch_bytes(uint32_t count, uint64_t total_in) {
+    const uint64_t m = streams_max_items(count, total_in);
+    return streams_slots_bytes(m) + sbk::k7_meta_bytes(count, m);
+}
+
+int sb_compress_streams_device_ws(const uint8_t* const* d_in_ptrs, const uint64_t* d_in_lens, uint32_t count,
+                                  uint64_t total_in, uint8_t* d_out, uint64_t cap, uint64_t* d_out_offs,
+                                  sb_error* d_statuses, sb_frame_result* d_result, void* scratch, uint64_t scratch_bytes,
+                                  void* stream, sb_error* err) {
+    if ((count && (!d_in_ptrs || !d_in_lens)) || (!d_out && cap) || !d_out_offs || !d_result || !scratch) return fail(err, SB_E_INVALID);
+    const uint64_t m = streams_max_items(count, total_in);
+    if (m > 0xFFFFFFFFull) return fail(err, SB_E_INVALID, m, 0xFFFFFFFFull);   // K1 counts units in 32 bits
+    const uint64_t need = sb_compress_streams_scratch_bytes(count, total_in);
+    if (scratch_bytes < need) return fail(err, SB_BUFFER_TOO_SMALL, scratch_bytes, need);
+    Ctx* c;
+    int rc = get_ctx(&c, err);
+    if (rc) return rc;
+    sbk::StreamsPlan p;
+    memset(&p, 0, sizeof p);
+    p.in_ptrs = d_in_ptrs; p.in_lens = d_in_lens; p.count = count; p.max_items = (uint32_t)m; p.total_in = total_in;
+    p.slots = (uint8_t*)align_up((size_t)scratch, 256);
+    sbk::k7_carve_meta(p, p.slots + streams_slots_bytes(m));
+    p.out = d_out; p.cap = cap; p.out_offs = d_out_offs; p.statuses = d_statuses; p.result = d_result;
+    rc = compress_streams_run(*c, p, (cudaStream_t)stream, err);
+    if (rc) return rc;
+    ok(err);
+    return 0;
+}
+
+uint64_t sb_decompress_streams_scratch_bytes(uint32_t count) { return sbk::k7_dec_bytes(count); }
+
+int sb_decompress_streams_device_ws(const uint8_t* const* d_in_ptrs, const uint64_t* d_in_lens, uint32_t count,
+                                    uint8_t* d_out, uint64_t cap, uint64_t* d_out_offs, sb_error* d_statuses,
+                                    sb_frame_result* d_result, void* scratch, uint64_t scratch_bytes,
+                                    void* stream, sb_error* err) {
+    if ((count && (!d_in_ptrs || !d_in_lens || !d_statuses)) || (!d_out && cap) || !d_out_offs || !d_result || !scratch)
+        return fail(err, SB_E_INVALID);
+    if (scratch_bytes < sbk::k7_dec_bytes(count)) return fail(err, SB_BUFFER_TOO_SMALL, scratch_bytes, sbk::k7_dec_bytes(count));
+    Ctx* c;
+    int rc = get_ctx(&c, err);
+    if (rc) return rc;
+    sbk::StreamsDecPlan p;
+    memset(&p, 0, sizeof p);
+    p.in_ptrs = d_in_ptrs; p.in_lens = d_in_lens; p.count = count;
+    p.out = d_out; p.cap = cap; p.out_offs = d_out_offs; p.statuses = d_statuses; p.result = d_result;
+    sbk::k7_carve_dec(p, scratch);
+    rc = decompress_streams_run(*c, p, (cudaStream_t)stream, err);
+    if (rc) return rc;
+    ok(err);
+    return 0;
+}
+
+// Host form: waves as in sb_compress_batch_host_packed (H2D, K7 + K1, D2H on three streams, double buffered); a unit
+// larger than a wave gets a wave of its own. Every unit is checked up front, so a wave never fails on the device.
+int sb_compress_streams_host_packed(const uint8_t* in_base, const uint64_t* in_offs, const uint64_t* in_lens, size_t count,
+                                    uint8_t* out_base, uint64_t out_cap, uint64_t* out_offs, sb_error* err) {
+    if ((count && (!in_base || !in_offs || !in_lens || !out_base)) || !out_offs) return fail(err, SB_E_INVALID);
+    for (size_t i = 0; i < count; i++)
+        if (sb_max_compress_len(in_lens[i]) == 0) return fail(err, SB_TOO_BIG, in_lens[i], SB_MAX_INPUT);
+    Ctx* c;
+    int rc = get_ctx(&c, err);
+    if (rc) return rc;
+    Lane& l = c->lane[LANE_ENC];
+    std::lock_guard<std::mutex> lk(l.mu);
+    const std::vector<Wave> waves = plan_waves(in_lens, count, (const uint32_t*)nullptr);
+    auto stage_in = [&](size_t wi) -> int {
+        const Wave& w = waves[wi];
+        const int b = (int)(wi & 1);
+        CK(l.in[b].need(w.in_bytes + 64));
+        CK(l.ptrs_in[b].need(w.count * 8 + 8));
+        CK(l.caps[b].need(w.count * 8 + 8));
+        // pinned[b] was last read by the H2D of wave wi-2, whose kernels have completed (the loop below waited for them)
+        { int prc = need_pinned(l, b, w.count * 16 + 64, err); if (prc) return prc; }
+        uint64_t* ptrs = (uint64_t*)l.pinned[b];
+        uint64_t* lens = ptrs + w.count;
+        uint64_t at = 0;
+        size_t i = 0;
+        while (i < w.count) {                                      // host-contiguous units travel as one copy
+            size_t j = i;
+            uint64_t run = 0;
+            const uint64_t h0 = in_offs[w.first + i];
+            while (j < w.count && in_offs[w.first + j] == h0 + run) {
+                ptrs[j] = (uint64_t)(uintptr_t)(l.in[b].as<uint8_t>() + at + run); run += in_lens[w.first + j]; j++;
+            }
+            if (run) CK(cudaMemcpyAsync(l.in[b].as<uint8_t>() + at, in_base + h0, run, cudaMemcpyHostToDevice, l.s_h2d));
+            at += (run + 15) & ~(uint64_t)15;
+            i = j;
+        }
+        memcpy(lens, in_lens + w.first, w.count * 8);
+        CK(cudaMemcpyAsync(l.ptrs_in[b].p, ptrs, w.count * 8, cudaMemcpyHostToDevice, l.s_h2d));
+        CK(cudaMemcpyAsync(l.caps[b].p, lens, w.count * 8, cudaMemcpyHostToDevice, l.s_h2d));
+        CK(cudaEventRecord(l.ev_in[b], l.s_h2d));
+        return 0;
+    };
+    auto drain_all = [&]() { cudaStreamSynchronize(l.s_h2d); cudaStreamSynchronize(l.s_compute); cudaStreamSynchronize(l.s_d2h); };
+    uint64_t packed_at = 0;
+    if (!waves.empty()) { rc = stage_in(0); if (rc) return rc; }
+    for (size_t wi = 0; wi < waves.size(); wi++) {
+        const Wave& w = waves[wi];
+        const int b = (int)(wi & 1);
+        CK(cudaStreamWaitEvent(l.s_compute, l.ev_in[b], 0));
+        if (wi >= 2) CK(cudaStreamWaitEvent(l.s_compute, l.ev_out[b], 0));   // wave wi-2 (same buffers) fully drained
+        uint64_t worst = 0;
+        for (size_t k = 0; k < w.count; k++) worst += sb_max_compress_len(in_lens[w.first + k]);
+        const uint64_t m = streams_max_items((uint32_t)w.count, w.in_bytes);
+        CK(l.compact[b].need(worst + 64));
+        CK(l.slots[b].need(m * (size_t)sbk::kSlotStride));
+        CK(l.sws[b].need(sbk::k7_meta_bytes(w.count, m)));
+        CK(l.ptrs_out[b].need(w.count * 8 + 8));
+        sbk::StreamsPlan p;
+        memset(&p, 0, sizeof p);
+        p.in_ptrs = (const uint8_t* const*)l.ptrs_in[b].p; p.in_lens = l.caps[b].as<uint64_t>();
+        p.count = (uint32_t)w.count; p.max_items = (uint32_t)m; p.total_in = w.in_bytes;
+        p.slots = l.slots[b].as<uint8_t>();
+        p.result = sbk::k7_carve_meta(p, l.sws[b].p);
+        p.out = l.compact[b].as<uint8_t>(); p.cap = l.compact[b].cap; p.out_offs = l.ptrs_out[b].as<uint64_t>();
+        rc = compress_streams_run(*c, p, l.s_compute, err);
+        if (rc) { drain_all(); return rc; }
+        { int prc = need_pinned(l, 2 + b, w.count * 8 + 8 + sizeof(sb_frame_result) + 64, err); if (prc) { drain_all(); return prc; } }
+        sb_frame_result* pres = (sb_frame_result*)l.pinned[2 + b];
+        uint64_t* poffs = (uint64_t*)(pres + 1);
+        CK(cudaMemcpyAsync(pres, p.result, sizeof *pres, cudaMemcpyDeviceToHost, l.s_compute));
+        CK(cudaMemcpyAsync(poffs, p.out_offs, (w.count + 1) * 8, cudaMemcpyDeviceToHost, l.s_compute));
+        CK(cudaEventRecord(l.ev_k[b], l.s_compute));
+        if (wi + 1 < waves.size()) { rc = stage_in(wi + 1); if (rc) { drain_all(); return rc; } }   // overlaps the kernels above
+        CK(cudaEventSynchronize(l.ev_k[b]));
+        if (pres->status.code) { const sb_error e = pres->status; drain_all(); if (err) *err = e; return (int)e.code; }
+        const uint64_t run = poffs[w.count];
+        if (packed_at + run > out_cap) { drain_all(); return fail(err, SB_BUFFER_TOO_SMALL, out_cap, packed_at + run); }
+        for (size_t k = 0; k < w.count; k++) out_offs[w.first + k] = packed_at + poffs[k];
+        CK(cudaStreamWaitEvent(l.s_d2h, l.ev_k[b], 0));
+        if (run) CK(cudaMemcpyAsync(out_base + packed_at, l.compact[b].p, run, cudaMemcpyDeviceToHost, l.s_d2h));
+        CK(cudaEventRecord(l.ev_out[b], l.s_d2h));
+        packed_at += run;
+    }
+    out_offs[count] = packed_at;
     CK(cudaStreamSynchronize(l.s_d2h));
     CK(cudaStreamSynchronize(l.s_compute));
     ok(err);
